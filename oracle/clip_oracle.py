@@ -4,8 +4,8 @@ text_transformer_forward`; the model itself is open_clip's `CLIP`, of which the 
 utils/reward/open_clip/: `transformer.py` ResidualAttentionBlock :189-244, VisionTransformer :323-520, `model.py` CLIP).
 
 Functional, driven by an open_clip-format state_dict (the format of `open_clip_pytorch_model.bin`).  Pinned against the
-vendored open_clip `CLIP` class itself (tests/test_oracle_pin.py when /root/reference is mounted; oracle/make_golden_clip.py
-freezes its outputs into tests/golden/clip_tiny.npz).
+vendored open_clip `CLIP` class itself (oracle/make_golden_clip.py compares it with that class and freezes its outputs
+into tests/golden/clip_tiny.npz).
 """
 from __future__ import annotations
 

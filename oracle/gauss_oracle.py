@@ -9,9 +9,8 @@ A functional restatement in plain torch (CPU, fp32 like the reference's tables).
 the SDE solver comes from torchsde.BrownianTree upstream -- a pip dependency that is absent here; both
 this oracle and the reference (through oracle/refload.py) use oracle/brownian.py, see its header.
 
-Pinning: tests/test_oracle_pin.py runs this file against the real GaussianDiffusion / sigma_schedule
-classes whenever /root/reference is mounted; oracle/make_golden.py freezes the sigma tables and one
-sampled latent into tests/golden/gauss.npz.
+Pinning: oracle/make_golden.py runs this file against the real GaussianDiffusion / sigma_schedule
+classes and freezes the sigma tables and one sampled latent into tests/golden/gauss.npz.
 """
 from __future__ import annotations
 

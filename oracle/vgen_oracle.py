@@ -9,9 +9,9 @@ Each function cites the reference lines it follows (paths relative to the refere
 
 Pinning: the reference has no tests or golden vectors for this path (SURVEY.md section 4), so the
 oracle is pinned against the reference ITSELF, imported on CPU through oracle/refload.py:
-tests/test_oracle_pin.py compares every function here with the reference classes when
-/root/reference is mounted, and oracle/make_golden.py freezes reference outputs into tests/golden/ so
-the pin also holds where the reference is absent (the GPU box).
+oracle/make_golden.py and oracle/make_golden_pin.py run the reference classes next to every function
+here and freeze their outputs into tests/golden/, which tests/test_oracle_golden.py and
+tests/test_oracle_pin.py compare with, so the pin holds where the reference is absent.
 
 Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference legs may import
 this module.  The product (vgen_b200/) never does.

@@ -5,7 +5,7 @@ text is split by a regex into words / digits / punctuation runs, every UTF-8 byt
 and adjacent symbols are merged greedily by the rank of the pair in the published merge list
 (`bpe_simple_vocab_16e6.txt.gz`, OpenAI CLIP, MIT licence); ids = [<start_of_text>] + pieces + [<end_of_text>], zero
 padded / truncated to 77.  This file implements that published algorithm; ids are index work, so the bar is bit-exact
-(tests/test_host_logic.py compares with the reference's vendored tokenizer when it is mounted and with committed ids).
+(tests/test_host_logic.py compares with ids the reference's vendored tokenizer produced, stored under tests/golden/).
 
 The merge list is data, not code: it is looked up (a) at `VGEN_CLIP_BPE`, (b) inside an installed `open_clip` package,
 (c) in the reference tree on `sys.path` (`utils/reward/open_clip/`), the way the engines' own import finds it.
