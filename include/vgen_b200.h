@@ -152,6 +152,20 @@ int vgen_sinusoidal_embedding(const float* t, void* out, int64_t b, int64_t dim,
 int vgen_adaptive_avgpool(const void* x, void* y, int64_t nimg, int64_t h, int64_t w, int64_t c, int64_t oh, int64_t ow,
                           int silu_in, void* stream);
 
+/* ---- condition adapters (cond_adapter.cu) ------------------------------------------------------- */
+/* Stem of every VideoComposer condition adapter, unet_videolcm.py:296-302 (and :306-371, unet_tf2tv.py likewise):
+ * Conv2d(cin -> cout, 3x3, pad 1) -> SiLU -> AdaptiveAvgPool2d((oh, ow)) per frame, fused (mma.sync tensor cores; the
+ * full-resolution activation never leaves shared memory).  x: the condition in the reference layout [b][cin][f][h][w],
+ * contiguous, fp32 (x_is_f32 = 1) or fp16; cin 1..4.  wt: fp16 K-major [cout][round_up(9*cin, 16)] with
+ * k = (ky*3 + kx)*cin + ci, padded columns zero; bias fp32 [cout]; cout 8..64 in steps of 8.  out: fp16 channels-last
+ * [(b f)][oh][ow][cout].  Pool bins are PyTorch's adaptive ones; a bin may span at most 16 rows / 32 columns. */
+int vgen_cond_stem(const void* x, int x_is_f32, int64_t b, int64_t cin, int64_t f, int64_t h, int64_t w, const void* wt,
+                   const float* bias, int64_t cout, int64_t oh, int64_t ow, void* out, void* stream);
+/* `concat = concat + adapter_i(...)` over the adapters of one forward (unet_videolcm.py:598-699): out[r][c] =
+ * fp16(sum_i srcs[i][r][c]) with the sum in fp32, in the order given (1..8 fp16 sources, row stride ld_src). */
+int vgen_cond_sum(const void* const* srcs, int nsrc, int64_t rows, int64_t cols, int64_t ld_src, void* out, int64_t ld_out,
+                  void* stream);
+
 /* DiagonalGaussianDistribution.sample * scale_factor (autoencoder.py:85-90,211-225): moments fp16 [n][p][2*zc]
  * (mean | logvar, channels-last) + fp32 noise [n][zc][p] -> fp32 z [n][zc][p] */
 int vgen_vae_sample(const void* moments, const float* noise, float* z, int64_t n, int64_t zc, int64_t p, float scale,

@@ -1,6 +1,6 @@
 """vgen_b200 -- B200-native (sm_100a) implementation of the VGen sampling hot path:
-DiffusionDDIM.ddim_sample_loop -> UNetSD_T2VBase / UNetSD_I2VGen (and the VideoLCM / SR600 / HiGen
-variants) forward -> AutoencoderKL.decode,
+DiffusionDDIM.ddim_sample_loop -> UNetSD_T2VBase / UNetSD_I2VGen (and the VideoLCM / TFT2V / SR600 / HiGen
+variants, with the VideoComposer condition adapters) forward -> AutoencoderKL.decode,
 exposed under the reference's MODEL / DIFFUSION / AUTO_ENCODER registry names (`register()`).
 
 Every op of the path is a hand-written CUDA kernel in libvgen_b200.so (include/vgen_b200.h); this
@@ -11,7 +11,7 @@ from .registry import register  # noqa: F401
 
 
 def __getattr__(name):  # lazy: importing the package must not require torch.cuda
-    if name in ("UNetSD_T2VBase", "UNetSD_I2VGen", "UNetSD_VideoLCM", "UNetSD_SR600", "UNetSD_HiGen"):
+    if name in ("UNetSD_T2VBase", "UNetSD_I2VGen", "UNetSD_VideoLCM", "UNetSD_TFT2V", "UNetSD_SR600", "UNetSD_HiGen"):
         from . import unet
         return getattr(unet, name)
     if name == "AutoencoderKL":

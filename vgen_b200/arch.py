@@ -43,6 +43,8 @@ class UNetPlan:
     concat_dim: int
     use_fps_condition: bool
     context_embedding_depth: int = 0        # higen: depth of TextContextCrossTransformerMultiLayer
+    compositions: Tuple[str, ...] = ()      # videolcm / tft2v: config.video_compositions
+    inpainting: bool = True                 # videolcm / tft2v: 'mask' builds masked_embedding only when True
     input_blocks: List[List[Layer]] = field(default_factory=list)
     middle: List[Layer] = field(default_factory=list)
     output_blocks: List[List[Layer]] = field(default_factory=list)
@@ -50,7 +52,8 @@ class UNetPlan:
 
 def unet_plan(kind, in_dim=4, dim=512, y_dim=512, context_dim=512, out_dim=6, num_tokens=4, dim_mult=(1, 2, 3, 4),
               num_heads=None, head_dim=64, num_res_blocks=3, attn_scales=(1 / 2, 1 / 4, 1 / 8), temporal_attention=True,
-              use_fps_condition=False, concat_dim=8, context_embedding_depth=4, **_ignored) -> UNetPlan:
+              use_fps_condition=False, concat_dim=8, context_embedding_depth=4, compositions=(), inpainting=True,
+              **_ignored) -> UNetPlan:
     """Block layout for the given constructor kwargs (defaults are the reference's own)."""
     if not temporal_attention:
         raise NotImplementedError("temporal_attention=False is not on the sampling hot path")
@@ -64,7 +67,8 @@ def unet_plan(kind, in_dim=4, dim=512, y_dim=512, context_dim=512, out_dim=6, nu
     has_concat = kind in ("i2vgen", "videolcm")  # channels concatenated to x before the first conv
     plan = UNetPlan(kind, in_dim, dim, embed_dim, y_dim, context_dim, out_dim, head_dim, num_tokens,
                     concat_dim if has_concat else 0, use_fps_condition,
-                    context_embedding_depth if kind == "higen" else 0)
+                    context_embedding_depth if kind == "higen" else 0,
+                    tuple(compositions) if kind == "videolcm" else (), bool(inpainting))
     enc_dims = [dim * u for u in [1] + list(dim_mult)]
     dec_dims = [dim * u for u in [dim_mult[-1]] + list(dim_mult)[::-1]]
     shortcut = []
@@ -175,8 +179,45 @@ def _mlp(p, a, b, c):
     return _lin(p + "0.", b, a) + _lin(p + "2.", c, b)
 
 
+# VideoComposer condition adapters of UNetSD_VideoLCM / UNetSD_TFT2V in the reference's creation order
+# (unet_videolcm.py:295-372): composition -> (stem module, Transformer_v2 module, condition channels)
+ADAPTERS = (
+    ("depthmap", "depth_embedding", "depth_embedding_after", 1),
+    ("motion", "motion_embedding", "motion_embedding_after", 2),
+    ("canny", "canny_embedding", "canny_embedding_after", 1),
+    ("mask", "masked_embedding", "mask_embedding_after", 4),
+    ("sketch", "sketch_embedding", "sketch_embedding_after", 1),
+    ("single_sketch", "single_sketch_embedding", "single_sketch_embedding_after", 1),
+    ("local_image", "local_image_embedding", "local_image_embedding_after", 3),
+)
+
+
+def _transformer_v2(p, cd):
+    """Transformer_v2(heads=2, dim=cd, dim_head=cd, mlp_dim=cd, depth=1), unet_videolcm.py:121-141 (Attention :39-67,
+    FeedForward util.py:724-741 with mult 4)."""
+    e = p + "layers.0."
+    return (_norm(e + "0.norm.", cd) + _lin(e + "0.fn.to_qkv.", 2 * cd * 3, cd, False) + _lin(e + "0.fn.to_out.0.", cd, 2 * cd) +
+            _lin(e + "1.net.0.0.", cd * 4, cd) + _lin(e + "1.net.2.", cd, cd * 4))
+
+
+def _vcomposer_spec(plan: UNetPlan) -> Spec:
+    cd = plan.concat_dim
+    s: Spec = []
+    if "image" in plan.compositions:
+        s += _mlp("pre_image_condition.", plan.context_dim, plan.context_dim, plan.context_dim * plan.num_tokens)
+    for comp, stem, after, cin in ADAPTERS:
+        if comp not in plan.compositions:
+            continue
+        if comp != "mask" or plan.inpainting:   # masked_embedding is None without inpainting, its Transformer_v2 exists
+            s += _conv(stem + ".0.", cd * 4, cin, 3, 3) + _conv(stem + ".3.", cd * 4, cd * 4, 3, 3) + _conv(stem + ".5.", cd, cd * 4, 3, 3)
+        s += _transformer_v2(after + ".", cd)
+    return s
+
+
 def unet_spec(plan: UNetPlan) -> Spec:
     s: Spec = _mlp("time_embed.", plan.dim, plan.embed_dim, plan.embed_dim)
+    if plan.kind == "videolcm":
+        s += _vcomposer_spec(plan)
     if plan.kind == "i2vgen":
         cd = plan.concat_dim
         s += _mlp("context_embedding.", plan.y_dim, plan.embed_dim, plan.context_dim * plan.num_tokens)

@@ -64,15 +64,22 @@ def cfg_forward(model, xt, ts, model_kwargs, by_keyword=False):
     A vgen_b200 UNet (`cfg_batch = True`) evaluates both branches as ONE forward of batch 2b -- the same arithmetic
     per sample (batch entries never interact), half the launches, and two tiles per CTA pair on the low-resolution
     layers so their epilogue overlaps a main loop.  Any other callable (e.g. a reference model) gets the reference's
-    two separate calls.  VGEN_CFG_BATCH=0 disables the batching."""
+    two separate calls.  VGEN_CFG_BATCH=0 disables the batching.
+
+    A model may declare `cfg_shared_kwargs`: a keyword in that set whose two branches hold the SAME tensor object (the
+    VideoComposer engines pass one condition tensor to both branches) is passed once, at batch b, and the model applies
+    it to both halves of the batch-2b forward.  Equal values in distinct tensors are concatenated like any other input."""
     kc, ku = model_kwargs
     m = _unwrap(model)
     call = (lambda x, t, kw: model(x, t=t, **kw)) if by_keyword else (lambda x, t, kw: model(x, t, **kw))
     if getattr(m, "cfg_batch", False) and os.environ.get("VGEN_CFG_BATCH", "1") != "0" and kc.keys() == ku.keys():
+        shared = getattr(m, "cfg_shared_kwargs", ())
         merged = {}
         for k in kc:
             a, b = kc[k], ku[k]
-            if torch.is_tensor(a) and torch.is_tensor(b) and a.shape == b.shape and a.dtype == b.dtype and a.dim() >= 1 \
+            if k in shared and a is b and torch.is_tensor(a):
+                merged[k] = a
+            elif torch.is_tensor(a) and torch.is_tensor(b) and a.shape == b.shape and a.dtype == b.dtype and a.dim() >= 1 \
                     and a.size(0) == xt.size(0):
                 merged[k] = torch.cat([a, b], dim=0)
             elif a is None and b is None:

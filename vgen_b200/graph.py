@@ -118,8 +118,13 @@ class GraphCache:
         return ent
 
 
-def graphed(fn):
-    """Decorator for a SpecModule method whose tensor arguments fully determine its device work."""
+def graphed(fn=None, *, key=None):
+    """Decorator for a SpecModule method whose tensor arguments fully determine its device work.  `key` names the
+    method's graph cache (default: the method's own name)."""
+    if fn is None:
+        return lambda f: graphed(f, key=key)
+    name = key or fn.__name__
+
     @functools.wraps(fn)
     def wrapper(self, *args, **kwargs):
         W = self._packed
@@ -128,7 +133,7 @@ def graphed(fn):
             if self._packed is not None and enabled():   # it still counts as the first sighting of this signature
                 flat = GraphCache._flatten(args, kwargs)
                 if flat is not None:
-                    c = self._packed.setdefault("__graphs__", {}).setdefault(fn.__name__, GraphCache())
+                    c = self._packed.setdefault("__graphs__", {}).setdefault(name, GraphCache())
                     c.seen[flat[1]] = max(c.seen.get(flat[1], 0), 1)
             return out
         if (not enabled() or ops.PROF is not None or not getattr(self, "use_cuda_graph", True)
@@ -137,9 +142,9 @@ def graphed(fn):
         cache = W.get("__graphs__")
         if cache is None:
             cache = W["__graphs__"] = {}
-        c = cache.get(fn.__name__)
+        c = cache.get(name)
         if c is None:
-            c = cache[fn.__name__] = GraphCache()
+            c = cache[name] = GraphCache()
         return c.run(fn, self, args, kwargs)
     wrapper.__wrapped_eager__ = fn
     return wrapper

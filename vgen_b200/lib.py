@@ -74,6 +74,8 @@ _SIGNATURES = {
     "vgen_linear_small": [_vp, _i64, _i64, _i64, _vp, _vp, _i64, _vp, _i64, _vp, _i64, _i32, _i32, _vp],
     "vgen_sinusoidal_embedding": [_vp, _vp, _i64, _i64, _vp],
     "vgen_adaptive_avgpool": [_vp, _vp, _i64, _i64, _i64, _i64, _i64, _i64, _i32, _vp],
+    "vgen_cond_stem": [_vp, _i32, _i64, _i64, _i64, _i64, _i64, _vp, _vp, _i64, _i64, _i64, _vp, _vp],
+    "vgen_cond_sum": [ctypes.POINTER(ctypes.c_void_p), _i32, _i64, _i64, _i64, _vp, _i64, _vp],
     "vgen_vae_sample": [_vp, _vp, _vp, _i64, _i64, _i64, _f32, _vp],
     "vgen_ddim_step": [_vp, _vp, _vp, _vp, _i64, _f32, _vp, _i32, _vp, _vp],
     "vgen_cfg_combine": [_vp, _vp, _vp, _i64, _i64, _f32, _vp, _vp],

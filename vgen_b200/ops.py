@@ -548,6 +548,66 @@ def adaptive_avgpool(x, oh, ow, silu_in=False):
     return y
 
 
+def cond_stem_k(cin):
+    """K (row length) of the vgen_cond_stem weight matrix: 9*cin padded to a multiple of 16."""
+    return (9 * cin + 15) // 16 * 16
+
+
+def pack_cond_stem_weight(w):
+    """Conv2d weight [cout, cin, 3, 3] -> fp32 [cout, cond_stem_k(cin)] with k = (ky*3+kx)*cin + ci, padding zero."""
+    cout, cin = w.shape[0], w.shape[1]
+    wp = torch.zeros(cout, cond_stem_k(cin), dtype=torch.float32)
+    wp[:, :9 * cin] = w.detach().float().cpu().permute(0, 2, 3, 1).reshape(cout, 9 * cin)
+    return wp
+
+
+def cond_stem(x, w, bias, oh, ow):
+    """Conv2d(3x3, pad 1) + bias -> SiLU -> AdaptiveAvgPool2d((oh, ow)) of every frame of a condition, one kernel.
+
+    x [b, cin, f, H, W] contiguous CUDA fp32 or fp16 (the reference layout), cin 1..4; w fp16 [cout, cond_stem_k(cin)]
+    (pack_cond_stem_weight), bias fp32 [cout], cout 8..64 in steps of 8 -> fp16 channels-last [(b f), oh, ow, cout]."""
+    if not x.is_cuda or x.dim() != 5 or not x.is_contiguous() or x.dtype not in (torch.float32, torch.float16):
+        raise _l.VgenError("cond_stem: x must be a contiguous CUDA fp32/fp16 tensor [b, cin, f, H, W]")
+    b, cin, f, h, wd = x.shape
+    _chk16(w, "w")
+    cout = w.shape[0]
+    if w.dim() != 2 or w.shape[1] != cond_stem_k(cin) or not w.is_contiguous():
+        raise _l.VgenError(f"cond_stem: weight {tuple(w.shape)} must be contiguous [cout, {cond_stem_k(cin)}] for cin={cin}")
+    if bias.dtype != torch.float32 or not bias.is_contiguous() or bias.numel() != cout or not bias.is_cuda:
+        raise _l.VgenError("cond_stem: bias must be a contiguous CUDA fp32 tensor [cout]")
+    out = torch.empty(b * f, oh, ow, cout, device=x.device, dtype=torch.float16)
+    n = b * f
+    rc = _run("cond_stem", 2.0 * n * h * wd * 9 * cin * cout, x.element_size() * x.numel() + 2.0 * out.numel() + 2.0 * w.numel(),
+              lambda: _l.load().vgen_cond_stem(_p(x), 1 if x.dtype == torch.float32 else 0, b, cin, f, h, wd, _p(w), _p(bias),
+                                               cout, oh, ow, _p(out), _stream()),
+              tag=f"cin{cin} {n}x{h}x{wd} -> {oh}x{ow}x{cout}")
+    _l.check(rc, "vgen_cond_stem")
+    return out
+
+
+def cond_sum(srcs, out=None):
+    """fp16(sum of the fp16 [rows, cols] tensors `srcs`, accumulated in fp32 in list order), 1..8 sources."""
+    if not 1 <= len(srcs) <= 8:
+        raise _l.VgenError("cond_sum: 1..8 sources")
+    views = []
+    for i, s in enumerate(srcs):
+        _chk16(s, f"srcs[{i}]")
+        views.append(_rows_view(s, f"srcs[{i}]"))
+    rows, cols = views[0][0].shape
+    ld = views[0][1]
+    if any(v.shape != (rows, cols) or l != ld for v, l in views):
+        raise _l.VgenError("cond_sum: sources must share shape and row stride")
+    if out is None:
+        out = torch.empty(rows, cols, device=srcs[0].device, dtype=torch.float16)
+    o2, ldo = _rows_view(out, "out")
+    if o2.shape != (rows, cols):
+        raise _l.VgenError("cond_sum: out shape mismatch")
+    ptrs = (ctypes.c_void_p * len(srcs))(*[v.data_ptr() for v, _ in views])
+    rc = _l.load().vgen_cond_sum(ptrs, len(srcs), rows, cols, ld, _p(o2), ldo, _stream())
+    _l.check(rc, "vgen_cond_sum")
+    return out
+
+
 def ddim_step_(xt, y, u, coef7, guide_scale, mean_type_v=True, noise=None, x0_out=None):
     """In-place fused CFG + DDIM update of the fp32 latent xt; y/u fp16 model outputs (same layout).
     x0_out (optional, fp32 like xt) receives the predicted x0 (diffusion_ddim.py:241 returns it)."""

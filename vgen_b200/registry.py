@@ -58,7 +58,7 @@ USING_REFERENCE_REGISTRY = False
 
 
 def register(force_local: bool = False):
-    """Register the UNets (T2VBase, I2VGen, VideoLCM, SR600, HiGen), DiffusionDDIM(SR), AutoencoderKL and the three
+    """Register the UNets (T2VBase, I2VGen, VideoLCM, TFT2V, SR600, HiGen), DiffusionDDIM(SR), AutoencoderKL and the three
     FrozenOpenCLIP*Embedder classes under the reference's registry names.  Returns (MODEL, DIFFUSION, AUTO_ENCODER); the
     embedder registry is `vgen_b200.registry.EMBEDDER`."""
     global MODEL, DIFFUSION, AUTO_ENCODER, EMBEDDER, USING_REFERENCE_REGISTRY
@@ -66,7 +66,7 @@ def register(force_local: bool = False):
     from .clip import FrozenOpenCLIPEmbedder, FrozenOpenCLIPTextVisualEmbedder, FrozenOpenCLIPVisualEmbedder
     from .diffusion import DiffusionDDIM
     from .diffusion_gauss import DiffusionDDIMSR
-    from .unet import UNetSD_HiGen, UNetSD_I2VGen, UNetSD_SR600, UNetSD_T2VBase, UNetSD_VideoLCM
+    from .unet import UNetSD_HiGen, UNetSD_I2VGen, UNetSD_SR600, UNetSD_T2VBase, UNetSD_TFT2V, UNetSD_VideoLCM
 
     regs = None
     emb = None
@@ -90,7 +90,7 @@ def register(force_local: bool = False):
                                         "the reference's (utils.registry_class)" if USING_REFERENCE_REGISTRY else "local mirror")
     with warnings.catch_warnings():
         warnings.simplefilter("ignore")  # replacing the reference classes is the point
-        for cls in (UNetSD_T2VBase, UNetSD_I2VGen, UNetSD_VideoLCM, UNetSD_SR600, UNetSD_HiGen):
+        for cls in (UNetSD_T2VBase, UNetSD_I2VGen, UNetSD_VideoLCM, UNetSD_TFT2V, UNetSD_SR600, UNetSD_HiGen):
             MODEL.register_class()(cls)
         DIFFUSION.register_class()(DiffusionDDIM)
         DIFFUSION.register_class()(DiffusionDDIMSR)

@@ -1,7 +1,7 @@
-"""B200-native UNetSD_T2VBase / UNetSD_I2VGen / UNetSD_VideoLCM / UNetSD_SR600 / UNetSD_HiGen: same constructor
-arguments, state_dict keys and forward signatures as the reference classes (tools/modules/unet/unet_t2v.py:19-277,
-unet_i2vgen.py:19-346, unet_videolcm.py:188-760, unet_sr600.py:52-299, unet_higen.py:175-467), but the forward is a
-fixed-layout graph of libvgen_b200.so kernels.
+"""B200-native UNetSD_T2VBase / UNetSD_I2VGen / UNetSD_VideoLCM / UNetSD_TFT2V / UNetSD_SR600 / UNetSD_HiGen: same
+constructor arguments, state_dict keys and forward signatures as the reference classes (tools/modules/unet/unet_t2v.py:19-277,
+unet_i2vgen.py:19-346, unet_videolcm.py:188-760, unet_tf2tv.py:188-843, unet_sr600.py:52-299, unet_higen.py:175-467), but
+the forward is a fixed-layout graph of libvgen_b200.so kernels.
 
 Design (not a port of the reference's module tree):
   * activations stay fp16 channels-last [(b f), h, w, C] for the whole forward; the reference's dozens
@@ -91,13 +91,19 @@ class _UNetBase(SpecModule):
                                    num_tokens=num_tokens, dim_mult=tuple(dim_mult), num_heads=num_heads, head_dim=head_dim,
                                    num_res_blocks=num_res_blocks, attn_scales=tuple(attn_scales),
                                    temporal_attention=temporal_attention, use_fps_condition=use_fps_condition,
-                                   concat_dim=concat_dim, context_embedding_depth=context_embedding_depth)
+                                   concat_dim=concat_dim, context_embedding_depth=context_embedding_depth,
+                                   compositions=self._compositions(config), inpainting=inpainting)
         # attributes the reference exposes and engines read
         self.in_dim, self.dim, self.y_dim, self.context_dim, self.out_dim = in_dim, dim, y_dim, context_dim, out_dim
         self.embed_dim, self.num_tokens, self.head_dim = dim * 4, num_tokens, head_dim
         self.zero_y = zero_y
         self.use_fps_condition = self.plan.use_fps_condition
         self._build_params(arch.unet_spec(self.plan), arch.unet_zero_init)
+
+    @staticmethod
+    def _compositions(config):
+        """config.video_compositions of the VideoComposer-capable classes; () for the others."""
+        return ()
 
     # ------------------------------------------------------------------------------ weight packing
     def _pack(self):
@@ -199,6 +205,19 @@ class _UNetBase(SpecModule):
             norm(e + "0.norm."), lin(e + "0.fn.to_qkv.", bias=False), lin(e + "0.fn.to_out.0.")
             lin(e + "1.net.0.0."), lin(e + "1.net.2.")
             conv3("local_image_embedding.0.", cin_pad=8), conv3("local_image_embedding.3."), conv3("local_image_embedding.5.")
+        if self.plan.compositions:
+            if "image" in self.plan.compositions:
+                lin("pre_image_condition.0."), lin("pre_image_condition.2.")
+            for comp, stem, after, _cin in arch.ADAPTERS:
+                if comp not in self.plan.compositions:
+                    continue
+                if comp != "mask" or self.plan.inpainting:
+                    W[stem + ".0.w"] = _f16(ops.pack_cond_stem_weight(sd[stem + ".0.weight"]), dev)
+                    W[stem + ".0.b"] = _f32(sd[stem + ".0.bias"], dev)
+                    conv3(stem + ".3."), conv3(stem + ".5.")
+                e = after + ".layers.0."
+                norm(e + "0.norm."), lin(e + "0.fn.to_qkv.", bias=False), lin(e + "0.fn.to_out.0.")
+                lin(e + "1.net.0.0."), lin(e + "1.net.2.")
         if self.KIND == "higen":
             W["context_embedding.tokens"] = _f16(sd["context_embedding.tokens"][0], dev)
             for d in range(self.plan.context_embedding_depth):
@@ -374,6 +393,17 @@ class _UNetBase(SpecModule):
         g = ops.group_norm(x, W["out.0.g"], W["out.0.b"], 1e-5, True)
         return ops.conv2d_3x3(g, W["out.2.w"], bias=W["out.2.b"])
 
+    def _transformer_v2(self, tok, W, e, b, f, hw, cd):
+        """Transformer_v2 / TransformerV2(heads=2, dim=cd, dim_head=cd, mlp_dim=cd, depth=1) over the f frames of every pixel
+        (unet_videolcm.py:121-141, util.py:1396-1452): x = Attention(LN(x)) + x; x = FF(x) + x with FF = Linear, GELU,
+        Linear.  tok: [(b f h w), cd] frame-major per video; e: the prefix of layers.0."""
+        xn = ops.layer_norm(tok, W[e + "0.norm.g"], W[e + "0.norm.b"])
+        qkv = ops.linear_small(xn, W[e + "0.fn.to_qkv.w"]).view(b, f, hw, 6 * cd)
+        att = ops.attention_temporal(qkv[..., :2 * cd], qkv[..., 2 * cd:4 * cd], qkv[..., 4 * cd:], 2, cd)
+        tok = ops.linear_small(att.view(-1, 2 * cd), W[e + "0.fn.to_out.0.w"], W[e + "0.fn.to_out.0.b"], residual=tok)
+        hid = ops.linear_small(tok, W[e + "1.net.0.0.w"], W[e + "1.net.0.0.b"], gelu_out=True)
+        return ops.linear_small(hid, W[e + "1.net.2.w"], W[e + "1.net.2.b"], residual=tok)
+
     def _mlp(self, x, W, p):
         h = ops.linear_small(x, W[p + "0.w"], W[p + "0.b"])
         return ops.linear_small(h, W[p + "2.w"], W[p + "2.b"], silu_in=True)
@@ -449,14 +479,7 @@ class UNetSD_I2VGen(_UNetBase):
         ximg = self._small_conv(ximg, W, "local_image_concat.4.", act_silu=True)      # [(b f), h, w, cd]
         cd = ximg.shape[-1]
         # TransformerV2(heads=2, dim=cd, dim_head=cd): tokens are the f frames of one pixel (util.py:1396-1452)
-        e = "local_temporal_encoder.layers.0."
-        tok = ximg.view(-1, cd)
-        xn = ops.layer_norm(tok, W[e + "0.norm.g"], W[e + "0.norm.b"])
-        qkv = ops.linear_small(xn, W[e + "0.fn.to_qkv.w"]).view(b, f, h * w, 6 * cd)
-        att = ops.attention_temporal(qkv[..., :2 * cd], qkv[..., 2 * cd:4 * cd], qkv[..., 4 * cd:], 2, cd)
-        tok = ops.linear_small(att.view(-1, 2 * cd), W[e + "0.fn.to_out.0.w"], W[e + "0.fn.to_out.0.b"], residual=tok)
-        hid = ops.linear_small(tok, W[e + "1.net.0.0.w"], W[e + "1.net.0.0.b"], gelu_out=True)
-        tok = ops.linear_small(hid, W[e + "1.net.2.w"], W[e + "1.net.2.b"], residual=tok)
+        tok = self._transformer_v2(ximg.view(-1, cd), W, "local_temporal_encoder.layers.0.", b, f, h * w, cd)
         return ops.eltwise("scale", tok, s=2.0)   # "concat += _ximg" twice (:294-295), exact in fp16
 
     def _local_tokens(self, local_first, W, b, h, w):
@@ -509,33 +532,82 @@ class UNetSD_I2VGen(_UNetBase):
         return ops.pc_to_cp(out.view(b, f * h * w, self.out_dim), b, self.out_dim, f * h * w).view(b, self.out_dim, f, h, w)
 
 
+def _cfg_get(config, name, default=None):
+    if config is None:
+        return default
+    if isinstance(config, dict):
+        return config.get(name, default)
+    return getattr(config, name, default)
+
+
 class UNetSD_VideoLCM(_UNetBase):
-    """Drop-in for tools/modules/unet/unet_videolcm.py:188-189 (MODEL 'UNetSD_VideoLCM') on the text-to-video
-    path of configs/videolcm_t2v_infer.yaml (video_compositions == ['text']): `concat` stays all-zero
-    (:598), pre_image is an empty Sequential (:409,:705) and the context is the text tokens (:713-726).
-    The other compositions (depth / sketch / motion / ... adapters of the VideoComposer path) are outside
-    SURVEY.md section 8 and raise."""
+    """Drop-in for tools/modules/unet/unet_videolcm.py:188-189 (MODEL 'UNetSD_VideoLCM').
+
+    Text-to-video (configs/videolcm_t2v_infer.yaml, video_compositions == ['text']): `concat` stays all-zero (:598),
+    pre_image is an empty Sequential (:409,:705) and the context is the text tokens (:713-726).
+
+    VideoComposer (configs/videolcm_vcomposer_infer.yaml, tft2v_vcomposer_*.yaml): one adapter per spatial composition
+    (depthmap, motion, canny, mask, sketch, single_sketch, local_image; :294-372) fills the concat channels of the first
+    conv (:598-703), and 'image' appends pre_image_condition(image) as num_tokens context tokens (:743-745).  The
+    conditions do not depend on x, t or y, and the engines pass the same tensors to every step of a video, so:
+      * the adapter stage runs eagerly, outside the CUDA graph, and its [b*f*h*w, concat_dim] fp16 result is memoised
+        (strong reference + version counter + shape / stride / dtype of every condition tensor); a graph replay never
+        copies a full-resolution condition;
+      * a condition tensor that both CFG branches share is passed once (cfg_shared_kwargs, diffusion.cfg_forward) and
+        its concat rows are applied to both halves of the batch-2b forward.
+    `histogram` and `use_text_clip_vip_model` are not supported and raise."""
     KIND = "videolcm"
+    COMPOSITIONS = ("text", "image") + tuple(a[0] for a in arch.ADAPTERS)
+    # forward keyword -> composition, in the order the reference adds the adapters to `concat` (:599-699)
+    CONDITIONS = (("depth", "depthmap"), ("local_image", "local_image"), ("motion", "motion"), ("canny", "canny"),
+                  ("sketch", "sketch"), ("single_sketch", "single_sketch"), ("masked", "mask"))
+    cfg_shared_kwargs = frozenset(k for k, _ in CONDITIONS)
+    _POSITIONAL = ("y", "depth", "image", "motion", "local_image", "single_sketch", "masked", "canny", "sketch", "histogram",
+                   "fps", "video_mask", "focus_present_mask", "prob_focus_present", "mask_last_frame_num")
+
+    @staticmethod
+    def _compositions(config):
+        comps = tuple(_cfg_get(config, "video_compositions", None) or ["text"])
+        bad = [c for c in comps if c not in UNetSD_VideoLCM.COMPOSITIONS]
+        if "histogram" in comps:
+            raise NotImplementedError("vgen_b200 UNetSD_VideoLCM: the 'histogram' composition is not supported")
+        if bad:
+            raise NotImplementedError(f"vgen_b200 UNetSD_VideoLCM: unknown video_compositions {bad}")
+        if _cfg_get(config, "use_text_clip_vip_model", False):
+            raise NotImplementedError("vgen_b200 UNetSD_VideoLCM: use_text_clip_vip_model is not supported")
+        return comps
 
     def __init__(self, config=None, *args, **kwargs):
-        comps = list(getattr(config, "video_compositions", None) or (config or {}).get("video_compositions", ["text"]))
-        if comps != ["text"]:
-            raise NotImplementedError(f"vgen_b200 UNetSD_VideoLCM: video_compositions {comps} != ['text'] is not on the hot path")
         super().__init__(config, *args, **kwargs)
-        self.video_compositions = comps
+        self.video_compositions = list(self.plan.compositions)
         self.concat_dim = self.plan.concat_dim
+        self.inpainting = self.plan.inpainting
+        res = _cfg_get(config, "resolution", None)
+        self.resolution = list(res) if res is not None else None
+        if set(self.video_compositions) & {a[0] for a in arch.ADAPTERS} and self.resolution is None:
+            raise ValueError("UNetSD_VideoLCM: config.resolution is required for the spatial compositions (:270,:299)")
+        self.adapter_runs = 0      # adapter stages computed (memo misses), for tests and benchmarks
 
-    @graphed
+    def forward(self, x, t, *args, **kwargs):
+        if len(args) > len(self._POSITIONAL):
+            raise TypeError("forward: too many positional arguments")
+        bound = dict(zip(self._POSITIONAL, args))
+        if bound.keys() & kwargs.keys():
+            raise TypeError(f"forward: multiple values for {sorted(bound.keys() & kwargs.keys())}")
+        bound.update(kwargs)
+        if bound.get("histogram") is not None:
+            raise NotImplementedError("vgen_b200 UNetSD_VideoLCM: the 'histogram' condition is not supported")
+        conds = [(k, comp, bound[k]) for k, comp in self.CONDITIONS if bound.get(k) is not None]
+        if not conds and bound.get("image") is None:
+            return self._forward_text(x, t, *args, **kwargs)
+        return self._forward_vcomposer(x, t, bound, conds)
+
+    @graphed(key="forward")
     @torch.no_grad()
-    def forward(self, x, t, y=None, depth=None, image=None, motion=None, local_image=None, single_sketch=None,
-                masked=None, canny=None, sketch=None, histogram=None, fps=None, video_mask=None,
-                focus_present_mask=None, prob_focus_present=0., mask_last_frame_num=0, **kwargs):
+    def _forward_text(self, x, t, y=None, depth=None, image=None, motion=None, local_image=None, single_sketch=None,
+                      masked=None, canny=None, sketch=None, histogram=None, fps=None, video_mask=None,
+                      focus_present_mask=None, prob_focus_present=0., mask_last_frame_num=0, **kwargs):
         self._check_x(x, t)
-        for name, v in (("depth", depth), ("image", image), ("motion", motion), ("local_image", local_image),
-                        ("single_sketch", single_sketch), ("masked", masked), ("canny", canny), ("sketch", sketch),
-                        ("histogram", histogram)):
-            if v is not None:
-                raise NotImplementedError(f"vgen_b200 UNetSD_VideoLCM: condition '{name}' is not on the text-only hot path")
         W = self._packed or self._pack()
         b, c, f, h, w = x.shape
         emb = self._time_embedding(t, fps, W)
@@ -549,6 +621,131 @@ class UNetSD_VideoLCM(_UNetBase):
         xin = ops.cp_to_pc(x.contiguous(), b, c, f * h * w, c_pad=cpad).view(b * f, h, w, cpad)
         out = self._trunk(xin, emb, ctx, W, b, f)
         return ops.pc_to_cp(out.view(b, f * h * w, self.out_dim), b, self.out_dim, f * h * w).view(b, self.out_dim, f, h, w)
+
+    # ------------------------------------------------------------------------------ VideoComposer path
+    def _latent_of_resolution(self):
+        """Latent size the adapters produce: AdaptiveAvgPool2d((res[1]//2, res[0]//2)) then two stride-2 convs."""
+        ph, pw = self.resolution[1] // 2, self.resolution[0] // 2
+        s2 = lambda n: (n - 1) // 2 + 1  # noqa: E731
+        return ph, pw, s2(s2(ph)), s2(s2(pw))
+
+    def _check_conditions(self, x, conds, image):
+        b, _, f, h, w = x.shape
+        comps = set(self.video_compositions)
+        cb = None
+        for name, comp, v in conds:
+            if comp not in comps:
+                raise ValueError(f"UNetSD_VideoLCM: condition '{name}' given but '{comp}' is not in video_compositions")
+            if comp == "mask" and not self.inpainting:
+                raise ValueError("UNetSD_VideoLCM: 'masked' given to a model built with inpainting=False (:563)")
+            cin = next(a[3] for a in arch.ADAPTERS if a[0] == comp)
+            if not torch.is_tensor(v) or v.dim() != 5 or v.shape[1] != cin or v.shape[2] != f:
+                raise ValueError(f"UNetSD_VideoLCM: condition '{name}' must be [b, {cin}, {f}, H, W], got "
+                                 f"{tuple(v.shape) if torch.is_tensor(v) else type(v)}")
+            if not v.is_cuda or v.dtype not in (torch.float32, torch.float16):
+                raise ValueError(f"UNetSD_VideoLCM: condition '{name}' must be a CUDA fp32 or fp16 tensor")
+            if cb is None:
+                cb = v.shape[0]
+            if v.shape[0] != cb or b % cb:
+                raise ValueError(f"UNetSD_VideoLCM: condition batches must agree and divide the batch of x ({b})")
+        if conds:
+            _, _, lh, lw = self._latent_of_resolution()
+            if (lh, lw) != (h, w):
+                raise ValueError(f"UNetSD_VideoLCM: config.resolution {self.resolution} reduces the conditions to {lh}x{lw}, "
+                                 f"but the latent is {h}x{w}")
+        if image is not None:
+            if "image" not in comps:
+                raise ValueError("UNetSD_VideoLCM: condition 'image' given but 'image' is not in video_compositions")
+            if not torch.is_tensor(image) or image.shape[-1] != self.context_dim or image.numel() != b * self.context_dim:
+                raise ValueError(f"UNetSD_VideoLCM: image must hold one {self.context_dim}-wide embedding per video")
+
+    def _adapter(self, v, comp, W, f, hw):
+        _, stem, after, _ = next(a for a in arch.ADAPTERS if a[0] == comp)
+        ph, pw, _, _ = self._latent_of_resolution()
+        cd = self.concat_dim
+        z = ops.cond_stem(v.contiguous(), W[stem + ".0.w"], W[stem + ".0.b"], ph, pw)   # conv + SiLU + pool, [(b f), ph, pw, 4cd]
+        z = self._conv3x3_s2(z, W, stem + ".3.")
+        z = self._conv3x3_s2(z, W, stem + ".5.", act_silu=True)                       # [(b f), h, w, cd]
+        return self._transformer_v2(z.view(-1, cd), W, after + ".layers.0.", v.shape[0], f, hw, cd)
+
+    @staticmethod
+    def _memo_key(conds):
+        """Identity of the condition tensors: None when one cannot be tracked (inference-mode tensors have no version
+        counter), so such calls always recompute."""
+        key = []
+        for name, _, v in conds:
+            if v.is_inference():
+                return None
+            key.append((name, v, v._version, tuple(v.shape), v.stride(), v.dtype))
+        return key
+
+    @staticmethod
+    def _memo_hit(memo, key):
+        if memo is None or key is None or len(memo[0]) != len(key):
+            return False
+        return all(a[0] == b[0] and a[1] is b[1] and a[2:] == b[2:] for a, b in zip(memo[0], key))
+
+    @torch.no_grad()
+    def _adapter_concat(self, conds, W, f, hw):
+        """sum of the adapter outputs in the reference's order, fp32 accumulation, one fp16 rounding: [cb*f*hw, concat_dim]."""
+        key = self._memo_key(conds)
+        memo = W.get("__cond_memo__")
+        if self._memo_hit(memo, key):
+            return memo[1]
+        W.pop("__cond_memo__", None)
+        outs = [self._adapter(v, comp, W, f, hw) for _, comp, v in conds]
+        concat = outs[0] if len(outs) == 1 else ops.cond_sum(outs)
+        self.adapter_runs += 1
+        if key is not None:
+            W["__cond_memo__"] = (key, concat)
+        return concat
+
+    def _forward_vcomposer(self, x, t, bound, conds):
+        self._check_x(x, t)
+        image = bound.get("image")
+        self._check_conditions(x, conds, image)
+        W = self._packed or self._pack()
+        b, c, f, h, w = x.shape
+        concat = self._adapter_concat(conds, W, f, h * w) if conds else None
+        return self._forward_cond(x, t, concat=concat, y=bound.get("y"), image=image, fps=bound.get("fps"))
+
+    @graphed(key="forward_vcomposer")
+    @torch.no_grad()
+    def _forward_cond(self, x, t, concat=None, y=None, image=None, fps=None):
+        W = self._packed or self._pack()
+        b, c, f, h, w = x.shape
+        emb = self._time_embedding(t, fps, W)
+        if y is None:
+            if self.zero_y is None:
+                raise ValueError("y is None and no zero_y was given")
+            y = self.zero_y.to(x.device).repeat(b, 1, 1)
+        ctx = self._to_f16_rows(y)
+        if image is not None:                  # context = [y, pre_image_condition(image) as num_tokens tokens] (:743-745)
+            img = self._to_f16_rows(image.reshape(1, b, self.context_dim)).view(b, self.context_dim)
+            tok = self._mlp(img, W, "pre_image_condition.")                     # [b, num_tokens * context_dim]
+            ly, cdim = ctx.shape[1], self.context_dim
+            full = torch.empty(b, (ly + self.num_tokens) * cdim, device=x.device, dtype=torch.float16)
+            ops.copy2d(ctx.reshape(b, ly * cdim), full[:, :ly * cdim])
+            ops.copy2d(tok, full[:, ly * cdim:])
+            ctx = full.view(b, ly + self.num_tokens, cdim)
+        cin = self.plan.input_blocks[0][0].cin
+        cpad = ((cin + 7) // 8) * 8
+        xin = ops.cp_to_pc(x.contiguous(), b, c, f * h * w, c_pad=cpad).view(-1, cpad)
+        if concat is not None:                 # the condition rows of cb videos, applied to every group of cb videos of x
+            n, cd = concat.shape
+            for j in range(xin.shape[0] // n):
+                ops.copy2d(concat, xin[j * n:(j + 1) * n, c:c + cd])
+        out = self._trunk(xin.view(b * f, h, w, cpad), emb, ctx, W, b, f)
+        return ops.pc_to_cp(out.view(b, f * h * w, self.out_dim), b, self.out_dim, f * h * w).view(b, self.out_dim, f, h, w)
+
+
+class UNetSD_TFT2V(UNetSD_VideoLCM):
+    """Drop-in for tools/modules/unet/unet_tf2tv.py:188-189 (MODEL 'UNetSD_TFT2V', configs/tft2v_*_infer.yaml): the same
+    trunk, adapters and parameters as UNetSD_VideoLCM.  Its misc_dropout(y) (:727) is the identity at inference; a `t_w`
+    keyword is accepted and ignored."""
+
+    def forward(self, x, t, *args, t_w=None, **kwargs):
+        return super().forward(x, t, *args, **kwargs)
 
 
 class UNetSD_SR600(_UNetBase):
